@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the dense-LA hot path on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic input: one bf16 matmul 8192^3 per GPU (BASELINE
@@ -276,6 +276,21 @@ def check_matmul_samples(c, seed_a, seed_b, out, batches, n, rng, samples=16):
     return bool(worst <= 1e-2 and worst_abs <= 0.05), worst
 
 
+DUMP_ROWS = 1024                 # rows of C dumped over all ranks: 1024 x 8192 f32 = 32 MiB
+
+
+def dump_headline(c, out, rank, world, out_dir):
+    """Write what the headline's last timed step left in this rank's bf16 product C (batch `rank` of the [world, 8192, 8192]
+    output) as float32: the same seeded sample of DUMP_ROWS // world rows on every run, plus their row indices, so two builds
+    given the same arguments can be compared output for output."""
+    from cubecl_b200 import synth
+    rows = np.sort(np.random.default_rng(0).choice(N_MM, max(1, DUMP_ROWS // world), replace=False))
+    got = synth.bf16_bits_to_f32(out.to_numpy(c)[rows])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"matmul_bf16_8192_b{rank}.npy"), got)
+    np.save(os.path.join(out_dir, f"matmul_bf16_8192_b{rank}_rows.npy"), rows.astype(np.float64))
+
+
 def multi_gpu_parity(c, D, dist, e, world, ids, xs, reduce, TensorHandle):
     """Exact checks of the multi-GPU paths, on the record the driver keeps (runtime_tests/all_reduce.rs:5-62 is the model:
     integer-valued data, the reduced value identical on every rank and equal to the closed form):
@@ -371,7 +386,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--quick", action="store_true", help="headline + reduce only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the headline's timed steps, write a fixed sample of rows of its last product to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(3, args.warmup)
     if args.impl == "reference":
         return run_reference(args)
@@ -442,6 +463,8 @@ def main():
         clocks["remeasured"] = True
     c.flush()
     mm_kernel = c.last_kernel()                       # the entry point the timed launches ran (reported, not assumed)
+    if args.dump_outputs:                             # before the rows below overwrite `o`
+        dump_headline(c, o, e.rank, world, args.dump_outputs)
     value = world * FLOPS_MM * args.steps / (ms * 1e-3) / 1e12
     per_launch_ms = ms / args.steps
     per_gpu_tflops = FLOPS_MM / (per_launch_ms * 1e-3) / 1e12

@@ -1,7 +1,7 @@
 """Extract the golden vectors the reference's own tests hold for the dense-LA path into reference_golden.json.
 
-Run in the authoring container only (reads /root/reference, which does not exist on the GPU box):
-    python tests/golden/make_golden.py
+Given a checkout of tracel-ai/cubecl at 4057f39e (the tests only read the JSON this writes):
+    python tests/golden/make_golden.py <path to the cubecl checkout>
 The reference cannot be executed here (Rust, no toolchain), so the goldens are the LITERAL expected arrays and input
 generators written in its test sources; this script parses them so nothing is transcribed by hand.
 """
@@ -9,9 +9,9 @@ from __future__ import annotations
 
 import json
 import re
+import sys
 from pathlib import Path
 
-REF = Path("/root/reference")
 OUT = Path(__file__).resolve().parent / "reference_golden.json"
 NUM = r"-?\d+(?:\.\d*)?"
 
@@ -25,9 +25,9 @@ def literal_after(text: str, anchor: str, opener: str) -> tuple[list[float], int
     return nums, text.count("\n", 0, s) + 1
 
 
-def main() -> None:
-    cmma = (REF / "crates/cubecl-core/src/runtime_tests/cmma.rs").read_text()
-    sums = (REF / "examples/sum_things/src/lib.rs").read_text()
+def main(ref: Path) -> None:
+    cmma = (ref / "crates/cubecl-core/src/runtime_tests/cmma.rs").read_text()
+    sums = (ref / "examples/sum_things/src/lib.rs").read_text()
     gold = {"_generated_by": "tests/golden/make_golden.py", "_reference": "tracel-ai/cubecl @ 4057f39e"}
 
     v, line = literal_after(cmma, "pub fn test_simple_1_expected", "vec![")
@@ -83,4 +83,6 @@ def main() -> None:
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        raise SystemExit("usage: python tests/golden/make_golden.py <path to the cubecl checkout>")
+    main(Path(sys.argv[1]))
